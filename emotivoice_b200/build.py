@@ -56,10 +56,20 @@ def build(force=False, verbose=True):
             fcntl.flock(lock, fcntl.LOCK_UN)
 
 
+def up_to_date(dig=None):
+    """True when the in-tree library exists and was built from the current sources and flags.  Only reads, so callers that
+    must not write into the tree (bench.py) can check the library without building it."""
+    stamp = os.path.join(LIB_DIR, "build.stamp")
+    if not (os.path.exists(LIB_PATH) and os.path.exists(stamp)):
+        return False
+    with open(stamp) as f:
+        return f.read().strip() == (dig or _digest())
+
+
 def _build_locked(force, verbose):
     stamp = os.path.join(LIB_DIR, "build.stamp")
     dig = _digest()
-    if not force and os.path.exists(LIB_PATH) and os.path.exists(stamp) and open(stamp).read().strip() == dig:
+    if not force and up_to_date(dig):
         if verbose:
             print("emotivoice_b200.build: up to date (sources digest %s), not recompiled" % dig[:12], flush=True)
         return LIB_PATH

@@ -15,6 +15,21 @@ import torch
 
 MAX_WAV_VALUE = 32768.0      # models/hifigan/get_vocoder.py (imported by inference_am_vocoder_joint.py:20)
 
+# The int16 files truncate fp32 samples, so one ulp anywhere in the forward can move a sample by one LSB, and the fp32 bits of a
+# CPU forward depend on the thread count and on the vector ISA torch's kernels pick for the host.  Files that are compared bit for
+# bit are therefore computed with pinned CPU arithmetic: one thread, ATen's baseline kernels, MKL's conditional numerical
+# reproducibility mode and no oneDNN, which gives the same bits on any x86-64 host.  ATen and MKL read these variables when
+# they load, so they go into the environment of a fresh process, which then calls pin_cpu_math() first.
+PINNED_CPU_ENV = {"ATEN_CPU_CAPABILITY": "default", "MKL_CBWR": "COMPATIBLE", "OMP_NUM_THREADS": "1", "MKL_NUM_THREADS": "1"}
+
+
+def pin_cpu_math():
+    import os
+    if any(os.environ.get(k) != v for k, v in PINNED_CPU_ENV.items()) or torch.backends.cpu.get_cpu_capability() != "DEFAULT":
+        raise RuntimeError("pinned CPU arithmetic needs a process started with %s in its environment" % PINNED_CPU_ENV)
+    torch.set_num_threads(1)
+    torch.backends.mkldnn.enabled = False
+
 
 def synthetic_style_embedding(text, seed=1234, dim=768):
     """Stand-in for get_style_embedding(prompt, tokenizer, style_encoder) (:25-38): a vector that depends only on the text,

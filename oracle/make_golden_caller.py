@@ -3,7 +3,8 @@
     python oracle/make_golden_caller.py          (build container: needs /root/reference)
 
 Runs oracle/caller_loop.run_caller_loop with the UNMODIFIED reference ``JETSGenerator`` class on the reference's own
-data/inference/text (12 lines), token / speaker tables and config.yaml, with the seeded synthetic checkpoint, on the CPU.
+data/inference/text (12 lines), token / speaker tables and config.yaml, with the seeded synthetic checkpoint, on the CPU with
+pinned arithmetic (caller_loop.PINNED_CPU_ENV: the script re-executes itself with it), so the files are reproducible on any host.
 Writes tests/golden/caller_lines.json (the 12 lines + the two symbol tables restricted to the symbols they use -- data, so the
 test needs no reference tree) and tests/golden/caller_ref_pcm.npz (the reference's int16 output for every line, as sample
 counts + sha1, and the full waveform of the three shortest lines)."""
@@ -11,6 +12,7 @@ import hashlib
 import json
 import os
 import sys
+import zipfile
 
 import numpy as np
 import torch
@@ -22,7 +24,21 @@ from emotivoice_b200 import synth                           # noqa: E402
 from oracle import caller_loop, refshim                      # noqa: E402
 
 
+def save_npz_lzma(path, **arrays):
+    """np.savez_compressed with LZMA members and fixed member dates: about half the size for int16 audio, the same bytes on every
+    run; np.load reads it like any .npz."""
+    with zipfile.ZipFile(path, "w") as zf:
+        for k, a in arrays.items():
+            info = zipfile.ZipInfo(k + ".npy")
+            info.compress_type = zipfile.ZIP_LZMA
+            with zf.open(info, "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(a), allow_pickle=False)
+
+
 def main():
+    if any(os.environ.get(k) != v for k, v in caller_loop.PINNED_CPU_ENV.items()):
+        os.execve(sys.executable, [sys.executable] + sys.argv, dict(os.environ, **caller_loop.PINNED_CPU_ENV))
+    caller_loop.pin_cpu_math()
     ref_root = refshim.REF_ROOT
     lines = [l.rstrip("\n") for l in open(os.path.join(ref_root, "data", "inference", "text"), encoding="utf-8") if l.strip()]
     token2id = {t.strip(): i for i, t in enumerate(open(os.path.join(ref_root, "data", "youdao", "text", "tokenlist"), encoding="utf-8"))}
@@ -32,7 +48,6 @@ def main():
     conf = refshim.load_reference_config(len(token2id), len(speaker2id))
     from emotivoice_b200.config import default_config
     sd = synth.make_state_dict(default_config(len(token2id), len(speaker2id)))
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
     JETS = refshim.import_reference_jets()
     res = caller_loop.run_caller_loop(JETS, conf, sd, lines, token2id, speaker2id, torch.device("cpu"))
     gold = os.path.join(ROOT, "tests", "golden")
@@ -48,7 +63,7 @@ def main():
         digests[str(n)] = hashlib.sha1(a.tobytes()).hexdigest()
         if n in keep:
             arrays["pcm_%d" % n] = a
-    np.savez_compressed(os.path.join(gold, "caller_ref_pcm.npz"), **arrays)
+    save_npz_lzma(os.path.join(gold, "caller_ref_pcm.npz"), **arrays)
     with open(os.path.join(gold, "caller_ref_digests.json"), "w") as f:
         json.dump({"sha1_of_reference_int16": digests, "torch": torch.__version__}, f, indent=1)
     print("lines", len(res), "samples", arrays["n_samples"].tolist(), "kept", sorted(keep))

@@ -3,18 +3,21 @@
 CLASS) is run on the reference's own 12 lines of data/inference/text with only the class swapped:
 
 * fixtures (tests/golden/caller_*) come from the UNMODIFIED reference class (oracle/make_golden_caller.py);
-* on the CPU the oracle port, wrapped in the same class interface, must reproduce the reference's int16 files exactly;
+* on the CPU the oracle port, wrapped in the same class interface, must reproduce the reference's int16 files exactly (both
+  computed with pinned CPU arithmetic, oracle/caller_loop.PINNED_CPU_ENV, in a process of their own);
 * on the GPU ``emotivoice_b200.modules.JETSGenerator`` must produce the same number of samples for every line (identical
   durations) and int16 samples within 1 LSB of the reference's (fp32 rounding differences of ~1e-6 can flip a truncation)."""
 import hashlib
 import json
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN
+from conftest import GOLDEN, ROOT
 from emotivoice_b200 import synth
 from emotivoice_b200.config import default_config
 from oracle import caller_loop, jets_oracle as O
@@ -49,15 +52,38 @@ class OracleJETS:
         return O.jets_forward(self.sd, self.conf, **kw)
 
 
-def test_oracle_behind_the_caller_loop_reproduces_the_reference_files_exactly():
-    meta, pcm, dig = _fixture()
+def oracle_on_the_stored_lines():
+    """[(line number, int16 audio)] of the oracle behind the caller loop, for the lines whose full waveform the fixture keeps."""
+    meta, pcm, _ = _fixture()
     conf = default_config(meta["n_vocab"], meta["n_speaker"])
     sd = synth.make_state_dict(conf)
     short = [n for n in pcm["line_no"].tolist() if "pcm_%d" % n in pcm.files]
     lines = [meta["lines"][n - 1] for n in short]
     res = caller_loop.run_caller_loop(OracleJETS, conf, sd, lines, meta["token2id"], meta["speaker2id"], torch.device("cpu"))
     assert len(res) == len(short)
-    for (_, audio), n in zip(res, short):
+    return [(n, audio) for (_, audio), n in zip(res, short)]
+
+
+_ORACLE_CHILD = r"""
+import os, sys
+import numpy as np
+sys.path[:0] = [sys.argv[1], os.path.join(sys.argv[1], "tests")]
+from oracle import caller_loop
+caller_loop.pin_cpu_math()
+import test_caller_dropin
+np.savez(sys.argv[2], **{"pcm_%d" % n: a for n, a in test_caller_dropin.oracle_on_the_stored_lines()})
+"""
+
+
+def test_oracle_behind_the_caller_loop_reproduces_the_reference_files_exactly(tmp_path):
+    meta, pcm, dig = _fixture()
+    out = str(tmp_path / "oracle_pcm.npz")
+    subprocess.run([sys.executable, "-c", _ORACLE_CHILD, ROOT, out], env=dict(os.environ, **caller_loop.PINNED_CPU_ENV), check=True, timeout=900)
+    res = np.load(out)
+    short = [n for n in pcm["line_no"].tolist() if "pcm_%d" % n in pcm.files]
+    assert sorted(res.files) == sorted("pcm_%d" % n for n in short)
+    for n in short:
+        audio = res["pcm_%d" % n]
         assert audio.dtype == np.int16 and np.array_equal(audio, pcm["pcm_%d" % n])
         assert hashlib.sha1(audio.tobytes()).hexdigest() == dig[str(n)]
 

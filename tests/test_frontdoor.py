@@ -9,7 +9,8 @@ import torch
 
 from emotivoice_b200 import frontdoor as fd
 
-REF = "/root/reference"
+# byte copies of the reference's data/youdao/text/{tokenlist,speaker2} and data/inference/text (oracle/make_golden_tables.py)
+REF_TEXT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_text")
 
 
 def test_parse_and_encode_follow_the_reference_contract(tmp_path):
@@ -31,13 +32,12 @@ def test_parse_and_encode_follow_the_reference_contract(tmp_path):
         fd.parse_line("only|three|fields")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
 def test_reference_inference_fixture_parses_with_the_reference_tables():
-    t2i = fd.load_symbol_table(os.path.join(REF, "data/youdao/text/tokenlist"))
-    s2i = fd.load_symbol_table(os.path.join(REF, "data/youdao/text/speaker2"))
+    t2i = fd.load_symbol_table(os.path.join(REF_TEXT, "tokenlist"))
+    s2i = fd.load_symbol_table(os.path.join(REF_TEXT, "speaker2"))
     assert len(t2i) == 502 and t2i["_"] == 0 and t2i["<sos/eos>"] == 1
     lens = []
-    with open(os.path.join(REF, "data/inference/text")) as f:
+    with open(os.path.join(REF_TEXT, "inference_text"), encoding="utf-8") as f:
         for line in f:
             enc = fd.encode(fd.parse_line(line), t2i, s2i)
             assert enc is not None and enc[0][0] == 1 and enc[0].max() <= 416

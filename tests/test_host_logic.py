@@ -1,6 +1,7 @@
 """CPU-only checks of the host side: weight packing (the load-time re-layouts the kernels
 rely on), state-dict compatibility with the reference's names, the C-ABI library's exported
 symbols, and the fail-loudly behaviour without a GPU."""
+import json
 import math
 import os
 import re
@@ -10,7 +11,7 @@ import torch
 import torch.nn.functional as F
 
 from emotivoice_b200 import synth, packing, _abi
-from emotivoice_b200.config import default_config, load_yaml_config
+from emotivoice_b200.config import default_config
 from oracle import jets_oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -149,12 +150,12 @@ def test_default_config_mirrors_reference_yaml_keys(conf):
     assert (c.hidden, c.n_heads, c.enc_layers, c.dec_layers, c.ffn_kernel, c.bert_dim) == (384, 8, 4, 4, 3, 768)
     assert [c.up_rates[i] for i in range(4)] == [8, 8, 2, 2] and [c.res_kernels[i] for i in range(3)] == [3, 7, 11]
     assert [c.res_dils[2][i] for i in range(3)] == [1, 3, 5]
-    ref_yaml = "/root/reference/config/joint/config.yaml"
-    if os.path.exists(ref_yaml):    # build container only
-        y = load_yaml_config(ref_yaml)
-        for k, v in conf.model.items():
-            assert y.model[k] == v, k
-        assert y.n_mels == conf.n_mels and y.segment_size == conf.segment_size
+    # the values of the reference's config/joint/config.yaml (oracle/make_golden_tables.py)
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_config.json")) as f:
+        y = json.load(f)
+    for k, v in conf.model.items():
+        assert y["model"][k] == v, k
+    assert y["n_mels"] == conf.n_mels and y["segment_size"] == conf.segment_size
 
 
 def test_synthetic_inputs_follow_the_input_contract():
